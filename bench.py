@@ -2,6 +2,7 @@
 """bench.py — inpainted frames/sec of FGT full inference at 432x240, T=10 (BASELINE.json configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl fgt_b200|reference|reference-gpu] [--config 2|3|4|5]
+                    [--dump-outputs DIR]
 
 Default (--config 2): a step is one Model.forward over one synthetic masked clip [1,10,3,240,432] (+flows,
 masks) with seeded random weights of the reference architecture. `value` is measured with the inputs already
@@ -12,6 +13,10 @@ no data-path collective), weak scaling, time = max over ranks. Additionally, at 
 split by frames over the ranks (FGT.enable_frame_sharding: the partitioning BASELINE.json's north_star names;
 exchange per temporal layer) and reported as strong scaling under `frame_sharded` (and, compactly, in
 `e2e.frame_sharded`, which the driver's record keeps).
+
+--dump-outputs DIR (default config and impl): after the timed steps, rank 0 writes the inpainted frames that the last
+timed step's Model.forward returned, [T,3,240,432] float32, to DIR/inpainted_frames.npy. Inputs and weights are seeded,
+so two builds run with the same arguments can be compared output for output.
 
 The other BASELINE configurations are separate lines: --config 3 (RAFT + LAFC at 480x864, T=20),
 --config 4 (432x240 T=80 clip = 16 windows of the driver's schedule, windows sharded over the ranks),
@@ -276,7 +281,12 @@ def main():
     ap.add_argument("--config", type=int, default=2, choices=[2, 3, 4, 5])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config != 2 or args.impl != "fgt_b200"):
+        ap.error("--dump-outputs is supported for the default --config 2 --impl fgt_b200 only")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -339,8 +349,10 @@ def main():
         total_ms = sum(a.elapsed_time(b) for a, b in evs)
         return parallel.max_over_ranks(total_ms, dev) / steps, launches
 
+    last = {}
+
     def step_device():
-        model(*devin)
+        last["out"] = model(*devin)   # kept for --dump-outputs: each step replaces the previous step's output
 
     def step_e2e():
         d = [h.to(dev, non_blocking=True) for h in host]
@@ -417,6 +429,11 @@ def main():
     sampler = ClockSampler(local_rank)
     sampler.start()
     ms_dev, launches = timed(step_device)
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "inpainted_frames.npy"), last["out"].float().cpu().numpy())
+    last.clear()
     ms_e2e_serial, _ = timed(step_e2e)
     ms_e2e, streamer = timed_streamed()
     clocks = sampler.stop()

@@ -5,17 +5,15 @@ from the script's directory before PYTHONPATH; dropin/run_driver.py reorders the
 reference tree (same package layout and the same import statements as tool/video_inpainting.py:1-33, marker modules
 instead of the real code), runs its driver through the launcher in a fresh interpreter and checks that every one
 of the six hot-path symbols comes from fgt_b200 while the modules the shims do not replace (RAFT.utils, other
-utils.*) still come from the reference tree. When /root/reference is present (build container), the same check
-runs against the real tree's import statements (the driver itself needs cvbase / imageio / skimage, which this
-image lacks, so its imports are replayed rather than executed).
+utils.*) still come from the reference tree. The same check also runs against the real driver's import statements
+and the real tree's module layout, both recorded from the original project in tests/golden/reference_driver_imports.json
+(the driver itself needs cvbase / imageio / skimage, so its imports are replayed rather than executed).
 """
 import json
 import os
 import subprocess
 import sys
 import textwrap
-
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LAUNCHER = os.path.join(ROOT, "dropin", "run_driver.py")
@@ -99,26 +97,28 @@ def test_plain_invocation_is_why_the_launcher_exists(tmp_path):
     assert not got["regionfill"].startswith("fgt_b200.")
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/tool"), reason="reference tree only exists in the build container")
 def test_real_reference_tree_imports(tmp_path):
-    """Replays the real driver's import statements (read from its source) for the hot-path modules under the
-    launcher's path order."""
-    src = open("/root/reference/tool/video_inpainting.py").read()
-    for stmt in ("from RAFT import RAFT", "import utils.region_fill as rf",
+    """Replays the real driver's import statements for the modules of its own tree (as recorded from its source)
+    under the launcher's path order, in a tree with the real tree's package layout (empty modules)."""
+    with open(os.path.join(ROOT, "tests", "golden", "reference_driver_imports.json")) as fh:
+        rec = json.load(fh)
+    for stmt in ("from RAFT import utils", "from RAFT import RAFT", "import utils.region_fill as rf",
                  "from utils.Poisson_blend_img import Poisson_blend_img",
                  "from get_flowNN_gradient import get_flowNN_gradient"):
-        assert stmt in src, stmt
+        assert stmt in rec["imports"], stmt
+    ref = str(tmp_path / "reference")
+    for rel in rec["modules"]:
+        p = os.path.join(ref, rel)
+        os.makedirs(os.path.dirname(p), exist_ok=True)
+        open(p, "w").close()
+    imports = "\n".join(rec["imports"])
     prog = textwrap.dedent(f'''
         import sys, json
         sys.path.insert(0, {os.path.join(ROOT, "dropin")!r})
         import run_driver
-        run_driver.setup_path("/root/reference/tool/video_inpainting.py")
-        sys.path += ["/root/reference", "/root/reference/FGT", "/root/reference/LAFC"]
-        from RAFT import utils
-        from RAFT import RAFT
-        import utils.region_fill as rf
-        from utils.Poisson_blend_img import Poisson_blend_img
-        from get_flowNN_gradient import get_flowNN_gradient
+        run_driver.setup_path({os.path.join(ref, rec["driver"])!r})
+        sys.path += [{ref!r}, {os.path.join(ref, "FGT")!r}, {os.path.join(ref, "LAFC")!r}]
+        exec({imports!r})
         from importlib import import_module
         fgt = import_module("FGT.models.model"); lafc = import_module("LAFC.models.lafc")
         print("RESULT " + json.dumps({{"RAFT": RAFT.__module__, "regionfill": rf.regionfill.__module__,
@@ -128,4 +128,4 @@ def test_real_reference_tree_imports(tmp_path):
     got = _run([sys.executable, "-c", prog], str(tmp_path))
     for key in ("RAFT", "regionfill", "Poisson_blend_img", "get_flowNN_gradient", "FGT.Model", "LAFC.Model"):
         assert got[key].startswith("fgt_b200."), (key, got[key])
-    assert got["RAFT.utils"].startswith("/root/reference/RAFT/utils")
+    assert got["RAFT.utils"].startswith(os.path.join(ref, "RAFT", "utils"))

@@ -37,7 +37,7 @@ def test_raft_state_dict_contract_and_dataparallel_roundtrip():
     got = model.state_dict()
     assert set(got.keys()) == set(sd.keys()) and len(got) == 179
     for k, v in sd.items():
-        assert torch.equal(got[k], v), k
+        assert torch.equal(got[k].cpu(), v), k   # DataParallel moves the module to cuda:0 when a GPU is present
     with pytest.raises(RuntimeError):
         model(*synth.raft_inputs(seed=0, H=64, W=64), iters=1, test_mode=True)  # CPU tensors: no fallback
     with pytest.raises(ValueError):

@@ -256,10 +256,9 @@ def run(args, rank, local_rank, world, out):
 
         sampler.start()
         l0 = lib.COUNTERS["launches"]
-        steps, warm = max(3, args.steps // 4), 3
-        ms = parallel.max_over_ranks(_events(lambda: step(False), steps, warm, flush, barrier), dev)
-        launches = (lib.COUNTERS["launches"] - l0) // (steps + warm)
-        ms_e2e = parallel.max_over_ranks(_events(lambda: step(True), max(2, steps // 2), 1, flush, barrier), dev)
+        ms = parallel.max_over_ranks(_events(lambda: step(False), args.steps, args.warmup, flush, barrier), dev)
+        launches = (lib.COUNTERS["launches"] - l0) // (args.steps + args.warmup)
+        ms_e2e = parallel.max_over_ranks(_events(lambda: step(True), max(2, args.steps // 2), 1, flush, barrier), dev)
         clocks = sampler.stop()
         model.net.enable_cuda_graph(False)
         ids = wins[0]
